@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the rasterizer hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -192,7 +192,8 @@ def make_inputs(B, rank):
 
 
 # ------------------------------------------------------------------------------------------------ step functions
-def ours_step(faces, tex, grad):
+def ours_step(faces, tex, grad, keep=None):
+    """`keep`: a dict that receives the rendered image (for --dump-outputs)"""
     import neural_renderer_b200 as nr
     w = WORKLOAD
     faces.grad = None
@@ -201,7 +202,37 @@ def ours_step(faces, tex, grad):
     img.backward(grad)  # upstream gradient dL/dI = grad, i.e. L = sum(I * grad)
     with torch.no_grad():
         loss = (img * grad).sum()
+    if keep is not None:
+        keep["image"] = img.detach()
     return loss
+
+
+DUMP_BYTES = 64 * 10 ** 6
+NPY_HEADER = 128  # bytes np.save puts before the data of a 1- to 4-dimensional float32 array
+
+
+def dump_outputs(out_dir, image, grad_faces, grad_textures):
+    """--dump-outputs: what one headline step hands its caller, as float32 .npy files, at most DUMP_BYTES in all.
+    In that order, each of the image, grad_faces and grad_textures is written whole as <name>.npy when it fits what
+    is left of the budget, else as <name>_sample.npy: the elements of the flattened tensor at a fixed, seeded set of
+    indices, as many as fit.  Returns {file name: shape}."""
+    os.makedirs(out_dir, exist_ok=True)
+    shapes, written = {}, 0
+    for name, t in (("image", image), ("grad_faces", grad_faces), ("grad_textures", grad_textures)):
+        room = (DUMP_BYTES - written - NPY_HEADER) // 4
+        if room <= 0:
+            break
+        if t.numel() > room:
+            flat = t.reshape(-1)
+            idx = np.sort(np.random.default_rng(0).choice(flat.numel(), room, replace=False))
+            t, name = flat[torch.from_numpy(idx).to(flat.device)], name + "_sample"
+        path = os.path.join(out_dir, name + ".npy")
+        a = t.detach().float().cpu().numpy()
+        np.save(path, a)
+        written += os.path.getsize(path)
+        shapes[name + ".npy"] = list(a.shape)
+    assert written <= DUMP_BYTES, written
+    return shapes
 
 
 def ref_gpu_step(faces, tex, grad):
@@ -578,7 +609,12 @@ def main():
     ap.add_argument("--shared-faces", type=int, default=1000000)
     ap.add_argument("--shared-image", type=int, default=1024)
     ap.add_argument("--views-per-gpu", type=int, default=8)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the image, grad_faces and a fixed sample of grad_textures of the "
+                         "last headline step to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "headline"):
+        ap.error("--dump-outputs writes the outputs of the headline workload of --impl ours")
     args.warmup = max(args.warmup, 3)
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -640,8 +676,10 @@ def main():
         return ms
 
     # ---- headline: device-resident inputs
+    last = {} if args.dump_outputs else None
+
     def step():
-        ours_step(faces, tex, grad)
+        ours_step(faces, tex, grad, keep=last)
 
     ms, t0, t1 = timed_loop(step, args.steps, args.warmup, barrier)
     ms = reduce_max(ms)
@@ -649,6 +687,10 @@ def main():
     value = pixels * args.steps / (ms * 1e-3) / 1e6
     clocks = sampler.summary(t0, t1)
     sampler.stop()  # the poller thread takes the GIL every 2 ms: keep it out of the launch-bound measurements below
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        dumped = dump_outputs(args.dump_outputs, last["image"], faces.grad, tex.grad)
+    last = None
 
     # count our kernel launches of one step through the library's own accounting
     import neural_renderer_b200 as nr
@@ -728,6 +770,8 @@ def main():
         "gpu_launches": launches_per_step * args.steps,
         "gpu_launches_per_step": launches_per_step,
     }
+    if dumped:
+        out["dump_outputs"] = {"dir": args.dump_outputs, "files": dumped}
     del sub
 
     # ---- side measurements (rank 0, N = 1, outside the headline region)

@@ -123,32 +123,37 @@ def test_face_light_and_fill_back_vs_reference_kernels():
     """rasterize(face_light=..., textures_fill_back=True) against the reference's own kernels fed the materialised
     tensors (bit-exact colours; texture / light gradients through the chain rule of the materialisation)."""
     import neural_renderer as nr
-    import refhost
     from neural_renderer_b200 import synthetic
-    if not refhost.available(64, 200, 4, 0.1, 100, 1e-4, 1, 0, 0):
-        pytest.skip("reference kernels not built")
+    from refgolden import RefGolden
+    from test_gpu_parity import _reference
     dev = torch.device("cuda")
     B, F2 = 3, 100
     half = synthetic.triangle_soup(B, F2, seed=11)
     faces = torch.from_numpy(np.concatenate([half, half[:, :, ::-1].copy()], axis=1)).to(dev)  # reversed copies
     tex = torch.from_numpy(synthetic.random_textures(B, F2, 4, seed=12)).to(dev)
     light = (torch.rand((B, 2 * F2, 3), generator=torch.Generator().manual_seed(13)) * 1.5).to(dev)
-    tex_a = tex.clone().requires_grad_(True)
-    light_a = light.clone().requires_grad_(True)
-    full = torch.cat((tex_a, tex_a.permute(0, 1, 4, 3, 2, 5)), dim=1) * light_a[:, :, None, None, None, :]
-    ref = refhost.rasterize_rgbad(faces, full.detach().contiguous(), 64, False, 0.1, 100, 1e-4, [0.1, 0.2, 0.3], True, False, False)
-    g = torch.randn(ref["rgb"].shape, generator=torch.Generator().manual_seed(14)).to(dev)
-    gf_ref, gfull_ref = ref.backward(g, None, None)
-    full.backward(gfull_ref)
+    g = torch.randn((B, 3, 64, 64), generator=torch.Generator().manual_seed(14)).to(dev)
+    gold = RefGolden("glue_face_light_fill_back")
+    if gold.recording:
+        tex_a = tex.clone().requires_grad_(True)
+        light_a = light.clone().requires_grad_(True)
+        full = torch.cat((tex_a, tex_a.permute(0, 1, 4, 3, 2, 5)), dim=1) * light_a[:, :, None, None, None, :]
+        ref = _reference(gold, faces, full.detach().contiguous(), 64, False, 0.1, 100, 1e-4, [0.1, 0.2, 0.3], (1, 0, 0))
+        gf_ref, gfull_ref = ref.backward(g, None, None)
+        full.backward(gfull_ref)
+        gold.put("grad_faces", gf_ref)
+        gold.put("grad_tex", tex_a.grad)
+        gold.put("grad_light", light_a.grad)
+        gold.save()
     fa = faces.clone().requires_grad_(True)
     tb = tex.clone().requires_grad_(True)
     lb = light.clone().requires_grad_(True)
     img = nr.rasterize(fa, tb, 64, False, 0.1, 100, 1e-4, [0.1, 0.2, 0.3], face_light=lb, textures_fill_back=True)
     (img * g).sum().backward()
-    assert torch.equal(img.detach(), ref["rgb"])
-    assert rel_err(fa.grad.cpu(), gf_ref.cpu()) <= 1e-4
-    assert rel_err(tb.grad.cpu(), tex_a.grad.cpu()) <= 1e-5
-    assert rel_err(lb.grad.cpu(), light_a.grad.cpu()) <= 1e-5
+    assert gold.equal("rgb", img)
+    assert gold.rel_err("grad_faces", fa.grad) <= 1e-4
+    assert gold.rel_err("grad_tex", tb.grad) <= 1e-5
+    assert gold.rel_err("grad_light", lb.grad) <= 1e-5
 
 
 def test_face_lighting_kernels(teapot):
@@ -227,8 +232,8 @@ def test_bake_textures_kernel_bit_exact(cfg):
     """nr_b200_bake_textures == the C oracle == the reference's own kernel string (load_obj.py:88-137), bit for bit,
     NaN texels included."""
     import nr_oracle as o
-    import refbake
     from neural_renderer_b200 import io
+    from refgolden import RefGolden
     ts, H, W = cfg
     img, uv, upd, tex = _bake_inputs(ts, H, W, 301, seed=ts * 100 + H)
     got = io.bake_textures(img, uv, upd, ts, tex)
@@ -237,17 +242,19 @@ def test_bake_textures_kernel_bit_exact(cfg):
     assert ((got.view(np.uint32) == want.view(np.uint32)) | (np.isnan(got) & np.isnan(want))).all()
     assert np.isnan(got).sum() == 3 * int(upd.sum())
     assert np.array_equal(got[upd == 0], tex[upd == 0])
-    if refbake.available(ts, H, W):
+    # faces 0 and 1 have UVs of exactly 1: there the reference kernel reads one row past the image -- with weight
+    # 0, or, when (int)(pos_y + 1) rounds up past (int)pos_y + 1, with weight ~1 (undefined in the reference); the
+    # product addresses those taps inside the image, so only the in-bounds faces are compared
+    gold = RefGolden("glue_bake_ts%d_%dx%d" % cfg)
+    if gold.recording:
+        import refbake
+        assert refbake.available(ts, H, W), "reference bake kernel not built (oracle/build_ref.py)"
         dev = torch.device("cuda")
         ref = refbake.bake(torch.from_numpy(img).to(dev), torch.from_numpy(uv).to(dev), torch.from_numpy(upd).to(dev), ts,
                            torch.from_numpy(tex).to(dev)).cpu().numpy()
-        same = (got.view(np.uint32) == ref.view(np.uint32)) | (np.isnan(got) & np.isnan(ref))
-        # faces 0 and 1 have UVs of exactly 1: there the reference kernel reads one row past the image -- with weight
-        # 0, or, when (int)(pos_y + 1) rounds up past (int)pos_y + 1, with weight ~1 (undefined in the reference); the
-        # product addresses those taps inside the image, so only the in-bounds faces are compared
-        assert same[2:].all()
-    else:
-        pytest.skip("reference bake kernel not built (compared with the C oracle only)")
+        gold.put("textures_in_bounds", ref[2:], exact_only=True)
+        gold.save()
+    assert gold.equal("textures_in_bounds", got[2:])  # bit for bit, every NaN texel read as one NaN
 
 
 def test_load_obj_with_textures_and_render():

@@ -1,5 +1,6 @@
 """GPU parity tests: the CUDA product (through the public API -> C ABI) against
   (a) the re-hosted reference kernels (oracle/refhost.py, exact oracle: face_index_map bit-exact, values <= 1e-4),
+      through the digests of their results stored under tests/golden/ref (tests/refgolden.py),
   (b) the CPU oracle (oracle/nr_oracle.c) at sizes it finishes in seconds,
   (c) the committed golden fixtures of the reference's own tests,
   (d) size-independent properties at the BASELINE.json headline shape.
@@ -16,6 +17,7 @@ pytestmark = pytest.mark.gpu
 TOL = 1e-4
 
 from helpers import np_, rel_err, to_minibatch  # noqa: E402
+from refgolden import RefGolden  # noqa: E402
 
 
 def _skip_without_gpu():
@@ -74,6 +76,57 @@ def _grads(shape_src, seed):
     return g
 
 
+def _reference(gold, faces, tex, image_size, aa, near, far, eps, bg, flags):
+    """While `gold` records: the reference kernels' forward on these inputs, its maps put into `gold`; the result
+    (whose .backward gives the reference gradients) is returned.  None when the stored digests are compared."""
+    if not gold.recording:
+        return None
+    import refhost
+    dev = torch.device("cuda")
+    faces = torch.as_tensor(faces).to(dev)
+    tex = torch.as_tensor(tex).to(dev) if flags[0] else None
+    S = image_size * 2 if aa else image_size
+    assert refhost.available(S, faces.shape[1], tex.shape[2] if flags[0] else 0, near, far, eps, *flags), \
+        "reference kernels for this configuration were not built (oracle/build_ref.py)"
+    ref = refhost.rasterize_rgbad(faces, tex, image_size, aa, near, far, eps, bg, *flags)
+    gold.put("fim", ref.fn.face_index_map, exact_only=True)
+    gold.put("wmap", ref.fn.weight_map, exact_only=True)
+    for k in ("rgb", "alpha", "depth"):
+        if ref[k] is not None:
+            gold.put(k, ref[k], exact_only=not aa)
+    return ref
+
+
+def _record_backward(gold, ref, grads, flags):
+    """While `gold` records: the reference gradients for upstream `grads`, put into `gold`, which is saved."""
+    if gold.recording:
+        gf, gt = ref.backward(grads.get("rgb"), grads.get("alpha"), grads.get("depth"))
+        gold.put("grad_faces", gf)
+        if flags[0]:
+            gold.put("grad_tex", gt)
+        gold.save()
+
+
+def _compare_forward(gold, got, aa):
+    # face_index_map: bit-exact (ours is stored in image orientation, the reference's un-flipped)
+    assert gold.equal("fim", got["fim"].flip(1)), "face_index_map differs"
+    # the forward maps replay the reference's fp32 expression trees, so they are expected to match bit for bit
+    # (the contract only asks for 1e-4; the stricter check guards the pinned arithmetic of nr_math.cuh)
+    assert gold.equal("wmap", got["wmap"].permute(0, 2, 3, 1).flip(1)), "weight_map not bit-exact"
+    for k in ("rgb", "alpha", "depth"):
+        if k in gold:
+            if aa:
+                assert gold.rel_err(k, got[k]) <= TOL, k
+            else:
+                assert gold.equal(k, got[k]), "%s: values differ in the last bits" % k
+
+
+def _compare_backward(gold, got, flags):
+    assert gold.rel_err("grad_faces", got["grad_faces"]) <= TOL, "grad_faces"
+    if flags[0]:
+        assert gold.rel_err("grad_tex", got["grad_tex"]) <= TOL, "grad_textures"
+
+
 # (name, image_size, anti_aliasing, F, ts, (rgb, alpha, depth), near, far, eps, mesh kind, B)
 CASES = [
     ("tiny_all", 32, False, 64, 2, (1, 1, 1), 0.1, 100, 1e-4, "soup", 3),
@@ -91,34 +144,16 @@ CASES = [
 
 @pytest.mark.parametrize("case", CASES, ids=[c[0] for c in CASES])
 def test_forward_backward_vs_reference_kernels(case):
-    import refhost
     name, image_size, aa, F, ts, flags, near, far, eps, kind, B = case
-    S = image_size * 2 if aa else image_size
-    if not refhost.available(S, F, ts if flags[0] else 0, near, far, eps, *flags):
-        pytest.skip("reference kernels for this configuration were not built (oracle/build_ref.py)")
     faces, tex = _inputs(kind, B, F, ts, seed=zlib.crc32(name.encode()) % 1000)
     bg = (0.1, 0.3, 0.5) if name != "soup_all" else np.linspace(0.0, 0.9, B * 3).reshape(B, 3).astype(np.float32)
-    dev = torch.device("cuda")
-    ref = refhost.rasterize_rgbad(torch.from_numpy(faces).to(dev), torch.from_numpy(tex).to(dev) if flags[0] else None,
-                                  image_size, aa, near, far, eps, bg, *flags)
-    grads = _grads(ref, seed=99)
+    gold = RefGolden("parity_" + name)
+    ref = _reference(gold, faces, tex, image_size, aa, near, far, eps, bg, flags)
+    grads = _grads(_run_product(faces, tex, image_size, aa, near, far, eps, bg, flags), seed=99)
+    _record_backward(gold, ref, grads, flags)
     got = _run_product(faces, tex, image_size, aa, near, far, eps, bg, flags, grads)
-
-    # face_index_map: bit-exact (ours is stored in image orientation, the reference's un-flipped)
-    assert torch.equal(got["fim"].flip(1), ref.fn.face_index_map), "face_index_map differs"
-    # the forward maps replay the reference's fp32 expression trees, so they are expected to match bit for bit
-    # (the contract only asks for 1e-4; the stricter check guards the pinned arithmetic of nr_math.cuh)
-    assert torch.equal(got["wmap"].permute(0, 2, 3, 1).flip(1), ref.fn.weight_map), "weight_map not bit-exact"
-    for k in ("rgb", "alpha", "depth"):
-        if ref[k] is not None:
-            assert rel_err(np_(got[k]), np_(ref[k])) <= TOL, k
-            if not aa:
-                nbad = int((got[k] != ref[k]).sum().item())
-                assert nbad == 0, "%s: %d values differ in the last bits" % (k, nbad)
-    gf, gt = ref.backward(grads.get("rgb"), grads.get("alpha"), grads.get("depth"))
-    assert rel_err(np_(got["grad_faces"]), np_(gf)) <= TOL, "grad_faces"
-    if flags[0]:
-        assert rel_err(np_(got["grad_tex"]), np_(gt)) <= TOL, "grad_textures"
+    _compare_forward(gold, got, aa)
+    _compare_backward(gold, got, flags)
 
 
 def _outside_box_wins(fim, faces, S):
@@ -138,26 +173,20 @@ def test_needle_faces(flags):
     """Needles whose long edges meet at 1e-7 .. 1e-4 rad win pixels BEYOND their tip in the reference (the fp32 edge
     tests of rasterize.py:309-311 accept a pixel centre on the needle's axis): the forward's conservative pixel box has
     to reach them (nr_bbox.cuh thin_face_margin).  Half of the faces are ordinary triangles that compete for the pixels."""
-    import refhost
     from neural_renderer_b200 import synthetic
     image_size, F, ts, B, near, far, eps = 64, 200, 4, 3, 0.1, 100, 1e-4
-    if not refhost.available(image_size, F, ts if flags[0] else 0, near, far, eps, *flags):
-        pytest.skip("reference kernels for this configuration were not built (oracle/build_ref.py)")
     faces = synthetic.triangle_soup(B, F, seed=11, z_range=(1.5, 3.0))
     faces[:, : F // 2] = synthetic.needle_faces(B, F // 2, image_size, seed=5)
     tex = synthetic.random_textures(B, F, ts, seed=3)
-    dev = torch.device("cuda")
     bg = (0.1, 0.3, 0.5)
-    ref = refhost.rasterize_rgbad(torch.from_numpy(faces).to(dev), torch.from_numpy(tex).to(dev) if flags[0] else None,
-                                  image_size, False, near, far, eps, bg, *flags)
-    ref_fim = np_(ref.fn.face_index_map)
-    assert _outside_box_wins(ref_fim, faces, image_size) >= 20, "the case does not exercise the thin-face margin"
+    gold = RefGolden("parity_needles_" + "".join(map(str, flags)))
+    _reference(gold, faces, tex, image_size, False, near, far, eps, bg, flags)
+    gold.save()
     got = _run_product(faces, tex, image_size, False, near, far, eps, bg, flags)
-    assert torch.equal(got["fim"].flip(1), ref.fn.face_index_map), "face_index_map differs"
-    assert torch.equal(got["wmap"].permute(0, 2, 3, 1).flip(1), ref.fn.weight_map), "weight_map not bit-exact"
-    for k in ("rgb", "alpha", "depth"):
-        if ref[k] is not None:
-            assert int((got[k] != ref[k]).sum().item()) == 0, k
+    # (the face_index_map equals the reference's bit for bit, so the product's map shows the reference's winners)
+    _compare_forward(gold, got, False)
+    assert _outside_box_wins(np_(got["fim"].flip(1)), faces, image_size) >= 20, \
+        "the case does not exercise the thin-face margin"
 
 
 @pytest.mark.parametrize("case", [c for c in CASES if c[0] in ("tiny_all", "soup_all", "npot_all", "aa_all")],
@@ -300,9 +329,6 @@ def test_golden_known_answer_gradients(kat, mode):
 def test_teapot_renderer_defaults_vs_reference_kernels(teapot):
     """BASELINE.json config 2 shape: teapot through Renderer defaults (fill_back, anti-aliasing, lighting), fwd+bwd."""
     import neural_renderer as nr
-    import refhost
-    if not refhost.available(512, 4928, 4, 0.1, 100, 1e-3, 1, 0, 0):
-        pytest.skip("reference kernels not built")
     dev = torch.device("cuda")
     v, f = teapot
     B = 2
@@ -316,19 +342,20 @@ def test_teapot_renderer_defaults_vs_reference_kernels(teapot):
     tx = torch.cat((tex, tex.permute(0, 1, 4, 3, 2, 5)), dim=1)
     tx = nr.lighting(nr.vertices_to_faces(vertices, fi), tx)
     faces = nr.vertices_to_faces(nr.perspective(nr.look_at(vertices, r.eye)), fi).contiguous()
-    ref = refhost.rasterize_rgbad(faces, tx.contiguous(), 256, True, 0.1, 100, 1e-3, [0, 0, 0], True, False, False)
-    g = torch.randn(ref["rgb"].shape, generator=torch.Generator().manual_seed(2)).to(dev)
+    gold = RefGolden("parity_teapot_renderer_defaults")
+    ref = _reference(gold, faces, tx.contiguous(), 256, True, 0.1, 100, 1e-3, [0, 0, 0], (1, 0, 0))
+    g = torch.randn((B, 3, 256, 256), generator=torch.Generator().manual_seed(2)).to(dev)
+    _record_backward(gold, ref, {"rgb": g}, (1, 0, 0))
     fa = faces.clone().requires_grad_(True)
     ta = tx.clone().requires_grad_(True)
     img = nr.rasterize(fa, ta, 256, True, 0.1, 100, 1e-3, [0, 0, 0])
     (img * g).sum().backward()
-    assert rel_err(np_(img), np_(ref["rgb"])) <= TOL
-    gf, gt = ref.backward(g, None, None)
-    assert rel_err(np_(fa.grad), np_(gf)) <= TOL
-    assert rel_err(np_(ta.grad), np_(gt)) <= TOL
+    assert gold.rel_err("rgb", img) <= TOL
+    assert gold.rel_err("grad_faces", fa.grad) <= TOL
+    assert gold.rel_err("grad_tex", ta.grad) <= TOL
     # and the facade itself produces that image
     img2 = r.render(vertices, faces_idx, tex)
-    assert rel_err(np_(img2), np_(ref["rgb"])) <= TOL
+    assert gold.rel_err("rgb", img2) <= TOL
 
 
 # ---------------------------------------------------------------------- properties at the headline shape (B=64)
@@ -388,21 +415,17 @@ def test_headline_gradient_checksums(headline):
 
 
 def test_headline_vs_reference_kernels(headline):
-    import refhost
-    if not refhost.available(256, 5000, 4, 0.1, 100, 1e-4, 1, 0, 0):
-        pytest.skip("reference kernels not built")
     faces, tex = headline
     B = 8  # the brute-force reference needs ~B * 3.3e8 face tests
-    dev = torch.device("cuda")
-    ref = refhost.rasterize_rgbad(torch.from_numpy(faces[:B]).to(dev), torch.from_numpy(tex[:B]).to(dev), 256, False,
-                                  0.1, 100, 1e-4, (0, 0, 0), True, False, False)
-    grads = _grads(ref, seed=99)
-    got = _run_product(faces[:B], tex[:B], 256, False, 0.1, 100, 1e-4, (0, 0, 0), (1, 0, 0), grads)
-    assert torch.equal(got["fim"].flip(1), ref.fn.face_index_map)
-    assert rel_err(np_(got["rgb"]), np_(ref["rgb"])) <= TOL
-    gf, gt = ref.backward(grads["rgb"], None, None)
-    assert rel_err(np_(got["grad_faces"]), np_(gf)) <= TOL
-    assert rel_err(np_(got["grad_tex"]), np_(gt)) <= TOL
+    args = (faces[:B], tex[:B], 256, False, 0.1, 100, 1e-4, (0, 0, 0), (1, 0, 0))
+    gold = RefGolden("parity_headline8")
+    ref = _reference(gold, *args)
+    grads = _grads(_run_product(*args), seed=99)
+    _record_backward(gold, ref, grads, (1, 0, 0))
+    got = _run_product(*args, grads)
+    assert gold.equal("fim", got["fim"].flip(1))
+    assert gold.equal("rgb", got["rgb"])  # bit-exact, as at every anti-aliasing-off shape
+    _compare_backward(gold, got, (1, 0, 0))
 
 
 def test_vertices_to_faces_kernels(teapot):

@@ -3,7 +3,6 @@ load_obj.py:8-197).  The fixture under tests/golden/textured is synthetic (tests
 import os
 
 import numpy as np
-import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 OBJ = os.path.join(ROOT, "tests", "golden", "textured", "quads.obj")
@@ -93,25 +92,3 @@ def test_textured_model_renders_like_the_reference_snapshot(monkeypatch):
     diff = np.abs(mine - ref)
     assert diff.mean() < 0.5 and diff.max() < 16.0, (diff.mean(), diff.max())   # observed 0.13 / 4.4 grey levels
 
-
-REF_DATA = os.path.join(os.environ.get("NR_REFERENCE_ROOT", "/root/reference"), "tests", "data")
-
-
-@pytest.mark.skipif(not os.path.exists(os.path.join(REF_DATA, "1cde62b063e14777c9152a706245d48", "model.obj")),
-                    reason="the 7.5 MB car model lives only in the reference tree (build container)")
-def test_car_model_renders_like_the_reference_snapshot(monkeypatch):
-    """test_load_obj.py:42-53: the 54 293-face car (Kd colours only) through this loader and the oracle's Renderer
-    against tests/data/car.png -- read straight from the reference tree where it exists (too large to commit)."""
-    import nr_oracle as o
-    from PIL import Image
-    from neural_renderer_b200 import io
-    monkeypatch.setattr(io, "bake_textures", lambda image, uv, upd, ts, tex: o.bake_textures(image, uv, upd, ts, tex))
-    v, f, tex = io.load_obj(os.path.join(REF_DATA, "1cde62b063e14777c9152a706245d48", "model.obj"), load_texture=True)
-    assert f.shape == (54293, 3) and tex.shape == (54293, 4, 4, 4, 3) and np.isfinite(tex).all()
-    r = o.Renderer()
-    r.eye = o.get_points_from_angles(2, 15, 30)
-    img = np.asarray(r.render(v[None], f[None], tex[None])["rgb"])[0].transpose(1, 2, 0)
-    mine = (img - img.min()) / (img.max() - img.min()) * 255.0
-    ref = np.asarray(Image.open(os.path.join(REF_DATA, "car.png"))).astype(np.float32)[..., :3]
-    diff = np.abs(mine - ref)
-    assert diff.mean() < 0.5 and (diff > 8).mean() < 1e-3, (diff.mean(), diff.max())  # observed mean 0.08, max 25 on a few edge pixels
